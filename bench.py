@@ -2,7 +2,7 @@
 """bench.py -- dispatch LPs/sec on BASELINE.json's headline config (C2: wind+battery, 24 periods, 10 000
 synthetic LMP scenarios per GPU), one JSON line on rank 0.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU, weak scaling: 10 000 LPs per rank,
                                                             one all_gather of the objectives per step)
 
@@ -26,6 +26,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True                 # the benchmark writes nothing into the tree, which may be read-only
 
 T = 24
 BATCH = 10000
@@ -162,8 +163,9 @@ def cpu_config_run(name, procs=None):
     return idx, obj, dt, procs
 
 
-def run_configs(world, rank, dev, reps=3):
-    """every rank: its interleaved shard of each config, timed on the device (max over ranks), one all_gather per pass"""
+def run_configs(world, rank, dev, reps=3, dump=None):
+    """every rank: its interleaved shard of each config, timed on the device (max over ranks), one all_gather per pass;
+    `dump` (a dict) receives the full obj / status / iters of each config's last timed pass"""
     import torch
     import torch.distributed as dist
     from dispatches_b200 import solver as S, sweep
@@ -204,6 +206,8 @@ def run_configs(world, rank, dev, reps=3):
                      "ms": best, "lps": N / best * 1e3, "non_optimal": int((st != 0).sum()),
                      "iters_mean": float(it.mean()), "iters_max": int(it.max()), "launch": S.last_launch(),
                      "obj": full["obj"].cpu().numpy()}
+        if dump is not None:
+            dump.update({f"{name}_obj": res[name]["obj"], f"{name}_status": st, f"{name}_iters": it})
         sol.close()
         del cp, rp, out, full
         torch.cuda.empty_cache()
@@ -243,7 +247,14 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the C3/C4/C5 block")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed paths returned in their last step as DIR/<name>.npy (float64): C2_obj, "
+                         "C2_status, C2_iters of rank 0's batch and <config>_obj / _status / _iters of every config")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -317,6 +328,9 @@ def main():
     t_wall = time.perf_counter() - t_wall0
     launches = S.launch_count() - n0
     out = outs[(args.steps - 1) % len(outs)]
+    dump = {} if args.dump_outputs else None
+    if dump is not None:                      # copied now: the passes below write into the same buffers
+        dump.update(C2_obj=out.obj.cpu().numpy(), C2_status=out.status.cpu().numpy(), C2_iters=out.iters.cpu().numpy())
     step_ms = sum(a.elapsed_time(b) for a, b, _ in ev) + ev_tail[0].elapsed_time(ev_tail[1])
     kern_ms = sum(a.elapsed_time(c) for a, _, c in ev)
     tt = torch.tensor([step_ms, kern_ms], dtype=torch.float64, device=dev)
@@ -361,7 +375,7 @@ def main():
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     sus_ms = float(tt[0])
     sus_clocks = sus_sampler.stop() if rank == 0 else None
-    cfg_res = {} if args.no_configs else run_configs(world, rank, dev)
+    cfg_res = {} if args.no_configs else run_configs(world, rank, dev, dump=dump)
     status = out.status.cpu().numpy()
     iters = out.iters.cpu().numpy()
     stats = torch.tensor([float((status != 0).sum()), float(iters.sum()), float(iters.max())], dtype=torch.float64, device=dev)
@@ -376,6 +390,12 @@ def main():
         dist.destroy_process_group()
     if rank != 0:
         return
+    if dump is not None:
+        dump = {k: np.asarray(v, dtype=np.float64) for k, v in dump.items()}
+        assert sum(a.nbytes for a in dump.values()) <= 64 << 20
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, v in dump.items():
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), v)
     total = BATCH * world
     value = total * args.steps / (step_ms * 1e-3)
     peaks = {}
@@ -435,7 +455,7 @@ def main():
                     "    except Exception as e:\n"
                     "        print('cpu baseline of', name, 'failed:', e, file=sys.stderr)\n"
                     "np.savez(%r, **out)") % (str(ROOT), [] if args.no_configs else list(CONFIG_DEFS), outp)
-            rc = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=1500)
+            rc = subprocess.run([sys.executable, "-B", "-c", code], capture_output=True, text=True, timeout=1500)
             if rc.returncode == 0:
                 z = np.load(outp)
                 cpu = dict(ref=z["ref"], dt=float(z["dt"]), procs=int(z["procs"]), n=int(z["n"]))

@@ -37,8 +37,11 @@ def needs_build():
 
 def build(force=False, verbose=False):
     """Builds the library if sources are newer.  Serialised across processes with a file lock: under torchrun every rank
-    calls this at start-up and only the first one may run nvcc."""
+    calls this at start-up and only the first one may run nvcc.  An up-to-date library is returned without writing
+    anything, so that a built tree can be used read-only."""
     import fcntl
+    if not force and not needs_build():
+        return LIB
     with open(HERE / ".build.lock", "w") as lk:
         fcntl.flock(lk, fcntl.LOCK_EX)
         try:

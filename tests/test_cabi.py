@@ -81,6 +81,16 @@ def test_forced_rebuild_from_source():
     assert lib.exists() and lib.stat().st_mtime >= t0 - 1.0
 
 
+def test_up_to_date_build_writes_nothing(cuda_solver_lib):
+    """bench.py calls build() and may run from a read-only tree: with the library current, build() creates or changes no file"""
+    from dispatches_b200.csrc import build
+    lib = build.build()
+    (lib.parent / ".build.lock").unlink(missing_ok=True)
+    before = {p: p.stat().st_mtime_ns for p in lib.parent.iterdir()}
+    assert build.build() == lib
+    assert {p: p.stat().st_mtime_ns for p in lib.parent.iterdir()} == before
+
+
 def build_c_example(tmp_path):
     import shutil
     import subprocess
